@@ -261,6 +261,24 @@ def time_pipe(torch, dist, world, pipe, stream, steps, warmup, which=0):
     return float(t.item()), launches
 
 
+def dump_pipe_outputs(pipe, out_dir, budget_bytes=60_000_000):
+    """The JPEG files of the pipe's last run, as a caller fetches them: jpeg_sizes.npy (float64, bytes per image) and
+    jpeg_bytes.npy (float32, images x K): each file's bytes at K fixed relative offsets, drawn once from a seeded generator so
+    that files of equal length are sampled at equal positions; K is capped so that both arrays stay under budget_bytes."""
+    n = pipe.n
+    k = min(1 << 16, budget_bytes // (4 * n))
+    frac = np.sort(np.random.default_rng(0).random(k))
+    sizes = np.zeros(n, dtype=np.float64)
+    sample = np.zeros((n, k), dtype=np.float32)
+    for i in range(n):
+        f = np.frombuffer(pipe.fetch(i), dtype=np.uint8)
+        sizes[i] = f.size
+        sample[i] = f[(frac * f.size).astype(np.int64)]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "jpeg_sizes.npy"), sizes)
+    np.save(os.path.join(out_dir, "jpeg_bytes.npy"), sample)
+
+
 def jpeg_e2e(args, L, torch, dist, world, datas, params, threads, e2e_threads):
     # ---- end to end through the C-ABI with host buffers
     Be = args.e2e_batch
@@ -301,8 +319,9 @@ def jpeg_e2e_only(args, L, torch, dist, world, datas, params, threads, e2e_threa
     return {"value": e2e["value"], "ms_total": 0.0, "launches": 0, "roofline": None, "e2e": e2e, "not_settled": 0, "encoder_retries": 0, "out_bytes_per_image": 0, "in_bytes_per_image": 0}
 
 
-def jpeg_workload(args, L, torch, dist, world, rank, datas, params, lossless, threads, e2e_threads, with_kernels=True):
-    """Resident full-path rate (`value`), per-kernel table, and the C-ABI rate (`e2e`) of one JPEG re-encode configuration."""
+def jpeg_workload(args, L, torch, dist, world, rank, datas, params, lossless, threads, e2e_threads, with_kernels=True, dump_dir=None):
+    """Resident full-path rate (`value`), per-kernel table, and the C-ABI rate (`e2e`) of one JPEG re-encode configuration;
+    dump_dir: where rank 0 writes the outputs of the last timed step (dump_pipe_outputs)."""
     px = W4K * H4K
     B = args.batch
     work = [datas[i % len(datas)] for i in range(B)]
@@ -312,6 +331,8 @@ def jpeg_workload(args, L, torch, dist, world, rank, datas, params, lossless, th
     pipe = L.JpegPipe(work, params, group=args.group)
     ms_total, launches = time_pipe(torch, dist, world, pipe, stream, args.steps, args.warmup)
     sizes, not_settled, retries = pipe.finish()
+    if dump_dir and rank == 0:
+        dump_pipe_outputs(pipe, dump_dir)
     value = world * B * MP_PER_IMAGE * args.steps / (ms_total / 1e3)
     if args.only_value:
         if rank == 0:
@@ -454,7 +475,10 @@ def main():
     ap.add_argument("--only-e2e", action="store_true", help="diagnostics: skip the device-resident leg and the per-kernel table")
     ap.add_argument("--only-value", action="store_true", help="diagnostics: the device-resident leg only (prints a short JSON line)")
     ap.add_argument("--only-configs", action="store_true", help="diagnostics: skip configs[1]; prints {\"configs\": {...}} for the sub-records named by --configs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the JPEG files of configs[1]'s last timed step under DIR as .npy (rank 0's shard), to compare two builds output for output")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.only_e2e or args.only_configs):
+        ap.error("--dump-outputs needs the device-resident leg of configs[1]")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     rank, world, local_rank = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("LOCAL_RANK", 0))
     if args.impl == "reference":
@@ -493,7 +517,7 @@ def main():
 
     clocks = ClockSampler(local_rank)
     clocks.start()
-    r1 = None if args.only_configs else jpeg_workload(args, L, torch, dist, world, rank, datas, p, False, threads, e2e_threads)
+    r1 = None if args.only_configs else jpeg_workload(args, L, torch, dist, world, rank, datas, p, False, threads, e2e_threads, dump_dir=args.dump_outputs)
     clk = clocks.stop()
 
     sub = {}

@@ -10,7 +10,7 @@ import pytest
 
 from pngutil import frame_png, idat_stream, pil_pixels, pil_png, synth
 
-P0_FILTER_HISTOGRAM = [3, 28, 211, 8, 150]      # per-row filter types 0..4 of /root/reference/samples/p0.png (known answer)
+P0_FILTER_HISTOGRAM = [3, 28, 211, 8, 150]      # per-row filter types 0..4 of the reference's samples/p0.png (known answer)
 
 CT = {1: 0, 2: 4, 3: 2, 4: 6}     # channels -> PNG colour type
 
@@ -258,13 +258,10 @@ def test_palette_reduction_is_lossless_and_declines_when_it_should(L):
 
 
 def test_reference_fixture_p0_png_known_answers(L, O):
-    """SURVEY.md §8c KAT-4 on the reference's own fixture (read where it lies; skipped on a box without /root/reference): one IDAT
+    """SURVEY.md §8c KAT-4 on the reference's own fixture (its copy in tests/golden/reference_samples): one IDAT
     that inflates to 480,400 bytes (400 rows of 400 RGB pixels + filter bytes); the product's host decoder and the oracle's
     unfilter must both reproduce libpng's pixels; the file's row-filter histogram is the known answer recorded here."""
-    path = "/root/reference/samples/p0.png"
-    if not os.path.exists(path):
-        pytest.skip("reference fixture not present")
-    data = open(path, "rb").read()
+    data = open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_samples", "p0.png"), "rb").read()
     ihdr, idat, order = idat_stream(data)
     assert ihdr[:5] == (400, 400, 8, 2, 0) and order.count(b"IDAT") == 1
     filt = np.frombuffer(zlib.decompress(idat), dtype=np.uint8)
